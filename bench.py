@@ -3,24 +3,31 @@
 reference C linker beside every number.
 
 Contract (DESIGN.md §7):
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--skip a,b,...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--skip a,b,...] [--dump-outputs DIR]
 
   N = 1 (plain `python bench.py`): headline = BASELINE.json configs[1] (cfg2, the 32-scalar-op fused Elemwise+CAReduce graph
       over fp32 (4096,4096)); a "step" is one evaluation of the compiled function.
-        value     evals/s, inputs resident in HBM, device outputs: MEDIAN over >= 25 windows of K steps each (CUDA events)
+        value     evals/s, inputs resident in HBM, device outputs: exactly K timed steps, issued as one uninterrupted
+                  stream and split into min(--reps, K // 10) (at least one) consecutive windows by CUDA events; MEDIAN
+                  over the windows of ms/step.  The steps alternate two input sets; the last one always runs on the first set (seed 1).
         e2e       evals/s through `pytensor.function(..., mode="CUDA")` with pinned HOST inputs and NumPy outputs
         roofline  achieved HBM GB/s of the dominant kernel over MEASURED_PEAKS.json
         parity    CUDA outputs vs the reference C linker's outputs on the SAME 4096^2 arrays
       and, always on: `metric_graph` (the 265-node Elemwise+Gemm+Scan graph BASELINE.json's metric names, n=64 and
       n=4096, with the C linker beside it), `cfg3` (MLP 4096^3: tcgen05 bf16 and the fp32-accurate default mode),
-      `cfg4` (Scan T=1000), `sharded_logp` (cfg5 on one GPU) — each with parity at the benchmarked shape.
+      `cfg4` (Scan T=1000), `sharded_logp` (cfg5 on one GPU) — each with parity at the benchmarked shape.  These, `e2e`
+      and the per-node profile behind `roofline` time fixed step counts of their own: --steps sets the headline only.
   N > 1 (torchrun): headline = BASELINE.json configs[4] (cfg5): hierarchical logp+grad over world x 2^17 independent
       chains sharded along the batch axis, ONE all-reduce of the packed [logp, grads] (75 floats) per evaluation, issued
       from inside the captured CUDA graph.  value = world x evaluations/s of the per-GPU shard (weak scaling); the line
       also carries the 1-GPU base measured in the same run, a strong-scaling point (2^20 chains in total), parity of
       the collective against a host sum of the per-rank partials and of rank 0's partial against the C linker, the
-      N-rank collective self-test, and cfg2 replicas under `others`.
+      N-rank collective self-test, and cfg2 replicas under `others`.  Here the headline is --reps windows of K steps each,
+      with a barrier before every window so that the slowest rank bounds each one.
   --impl reference: the reference's own C linker (mode="CVM") on the host cores, same config strings (rank 0 only).
+  --dump-outputs DIR (N = 1): after the timed steps, the headline's outputs of the last timed step as DIR/e.npy and
+      DIR/r.npy (see dump_outputs), so that two builds can be compared output for output.  --impl reference dumps its
+      last step too, on the same first input set.
 """
 
 from __future__ import annotations
@@ -35,12 +42,30 @@ import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+# a run writes nothing into the source tree, not even __pycache__/ for the modules that build() never imported
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 
 B_LOCAL = 1 << 17      # chains per GPU of the sharded logp+grad graph (2^20 at 8 GPUs)
 PAR_ROWS = 512         # rows of the n=4096 metric graph the C linker evaluates for parity (rows are independent)
 N_ROWS, N_GROUPS, N_COV = 1024, 64, 8
+MIN_WINDOW_STEPS = 10  # each event recorded between two steps costs device time: keep it under ~1/10 of a window
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(dirname, named):
+    """Write each output as `dirname/<name>.npy`, in float64 if it was computed in float64 and float32 otherwise.  Each
+    output gets an equal share of DUMP_BYTES; a larger one is written as its elements at a fixed, seeded set of flat
+    indices (sorted), the same in every run, so that dumps of the same arguments compare element for element."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in named.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        keep = (DUMP_BYTES // len(named) - 1024) // a.itemsize  # 1 KiB of each share is left for the .npy header
+        if a.size > keep:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def _peaks():
@@ -215,6 +240,24 @@ def timed_windows(fn, steps, reps, sync, barrier=None):
     return out
 
 
+def timed_steps(fn, steps, windows, sync):
+    """`steps` calls `fn(0..steps-1)` issued back to back, split into `windows` (at most steps // MIN_WINDOW_STEPS, at
+    least one) consecutive windows of near-equal size by CUDA events on the VM stream, one synchronise at the end: the
+    device never waits for the host between windows.  Returns per-window ms/step."""
+    import torch
+
+    windows = max(1, min(windows, steps // MIN_WINDOW_STEPS))
+    bounds = [steps * w // windows for w in range(windows + 1)]
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(windows + 1)]
+    ev[0].record()
+    for w in range(windows):
+        for i in range(bounds[w], bounds[w + 1]):
+            fn(i)
+        ev[w + 1].record()
+    sync()
+    return [ev[w].elapsed_time(ev[w + 1]) / (bounds[w + 1] - bounds[w]) for w in range(windows)]
+
+
 def window_stats(ms):
     a = np.sort(np.asarray(ms, dtype=np.float64))
     return {"n": int(a.size), "median_ms": float(np.median(a)), "min_ms": float(a[0]), "max_ms": float(a[-1]),
@@ -250,8 +293,10 @@ def reference_arm(args, rank, world):
         f(*a)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        f(*a)
+        out = f(*a)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("e", "r"), out)))
     v = args.steps * scale / dt
     print(json.dumps({
         "impl": "reference", "metric": "fn evals/sec", "value": v, "unit": "evals/s", "n_gpus": args.gpus,
@@ -598,13 +643,23 @@ def bench_cfg2(args, pytensor, W, cuda_mode, dev, jit, torch, dist, world, rank,
             for i in range(16):
                 f_dev(*dev_args[i % 2])
             torch.cuda.synchronize()
-        ms_w = timed_windows(lambda i: f_dev(*dev_args[i % 2]), args.steps, reps, torch.cuda.synchronize, barrier)
+        last = [None]
+
+        def step(i):  # the two input sets alternate, and the last step runs on the first one
+            last[0] = f_dev(*dev_args[(args.steps - 1 - i) % 2])
+
+        barrier()
+        ms_w = timed_steps(step, args.steps, reps, torch.cuda.synchronize)
+        # the outputs are borrowed buffers that the next call overwrites: copy the last timed step's now
+        dumped = dict(zip(("e", "r"), (dev.to_host(o) for o in last[0]))) if args.dump_outputs else None
         t_end = time.perf_counter() + 0.6
         while time.perf_counter() < t_end:  # keep the same load up so that later nvidia-smi samples see it
             for i in range(64):
                 f_dev(*dev_args[i % 2])
             torch.cuda.synchronize()
     replayed = bool(ex.last_from_graph)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if dist is not None:
         t = torch.tensor(ms_w, device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -700,8 +755,11 @@ def bench_cfg2(args, pytensor, W, cuda_mode, dev, jit, torch, dist, world, rank,
                    "steps": e2e_steps, "windows": 5,
                    "pipeline": ("chunked H2D|kernel|D2H x%d" % len(f_host.vm.executor._chunk_plan["bounds"]))
                    if f_host.vm.executor.chunked_calls else "one-shot"},
-           "gpu_launches": launches_per_step * args.steps * reps, "roofline": roofline, "cpu_baseline": cpu, "parity": par,
-           "clocks": clocks.summary()}
+           "gpu_launches": launches_per_step * args.steps, "roofline": roofline, "cpu_baseline": cpu, "parity": par,
+           "clocks": clocks.summary(),
+           "timing": {"timed_steps": args.steps, "windows": len(ms_w),
+                      "statistic": "median over windows of ms/step; the windows split one uninterrupted run of the "
+                                   "timed steps (per window: max over ranks)"}}
     return rec
 
 
@@ -729,15 +787,21 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--n", type=int, default=4096)
-    ap.add_argument("--reps", type=int, default=25, help="timed windows of --steps steps each (median reported)")
+    ap.add_argument("--reps", type=int, default=25,
+                    help="N = 1: windows the --steps timed steps are split into (at most --steps // 10); N > 1: "
+                         "windows of --steps steps each (median reported)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip", default="", help="comma list of: metric,cfg3,cfg4,cfg5,k1,cfg2 (developer runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     skip = {s for s in args.skip.split(",") if s}
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs measures one GPU")
 
     if args.impl == "reference":
         reference_arm(args, rank, world)
@@ -780,9 +844,11 @@ def main():
                                                          "statistic": "median over windows (per window: max over ranks)"}}
 
     if world == 1:
-        c2 = bench_cfg2(args, pytensor, W, cuda_mode, dev, jit, torch, dist, world, rank, local_rank, cvm, reps, want_cpu)
+        c2 = bench_cfg2(args, pytensor, W, cuda_mode, dev, jit, torch, dist, world, rank, local_rank, cvm, args.reps,
+                        want_cpu)
         line = dict(base)
-        for k in ("value", "ms_per_step", "windows", "e2e", "gpu_launches", "roofline", "cpu_baseline", "parity", "clocks"):
+        for k in ("value", "ms_per_step", "windows", "e2e", "gpu_launches", "roofline", "cpu_baseline", "parity", "clocks",
+                  "timing"):
             line[k] = c2[k]
         torch.cuda.empty_cache()
         if "k1" not in skip:

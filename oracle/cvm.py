@@ -1,7 +1,7 @@
 """Reference oracle: the reference's own C linker (`mode="CVM"`, pytensor/compile/mode.py:511) on the host CPU.
 
-TEST INFRASTRUCTURE — see oracle/__init__.py.  The reference is imported from baseline/_ref (built by
-oracle/build_ref.sh from the read-only checkout); nothing here reads /root/reference at run time.
+TEST INFRASTRUCTURE — see oracle/__init__.py.  The reference is imported from oracle/_ref (built by
+oracle/build_ref.sh from a pytensor checkout); nothing here reads the checkout itself at run time.
 """
 
 from __future__ import annotations
@@ -27,7 +27,7 @@ def _find_blas():
 
 
 def configure(floatX=None):
-    """Set PYTENSOR_FLAGS (compile dir, BLAS) BEFORE pytensor is imported; import it from baseline/_ref."""
+    """Set PYTENSOR_FLAGS (compile dir, BLAS) BEFORE pytensor is imported; import it from oracle/_ref."""
     global _configured
     if not _configured:
         flags = [f for f in os.environ.get("PYTENSOR_FLAGS", "").split(",") if f]
@@ -51,7 +51,7 @@ def configure(floatX=None):
                 if ok and "blas__ldflags" not in keys:
                     flags.append(f"blas__ldflags=-L{d} -l:{lib}")
         os.environ["PYTENSOR_FLAGS"] = ",".join(flags)
-        ref = os.path.join(REPO, "baseline", "_ref")
+        ref = os.path.join(_HERE, "_ref")
         if "pytensor" not in sys.modules and os.path.isdir(os.path.join(ref, "pytensor")) and ref not in sys.path:
             sys.path.insert(0, ref)
         _configured = True

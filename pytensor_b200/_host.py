@@ -1,6 +1,6 @@
 """Locate the host framework.  PyTensor itself is NOT part of this repo: it is the host whose Linker plugin surface
-the backend implements.  Search order: an installed `pytensor`, the reference build in `baseline/_ref` (produced by
-oracle/build_ref.sh; git-ignored, travels with the gpurun snapshot), then the read-only checkout in /root/reference.
+the backend implements.  Search order: an installed `pytensor`, then the reference build in `oracle/_ref` (produced by
+oracle/build_ref.sh from `__graft_entry__.build()`; git-ignored).
 """
 
 from __future__ import annotations
@@ -10,7 +10,7 @@ import os
 import sys
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = [os.path.join(REPO, "baseline", "_ref"), "/root/reference"]
+CANDIDATES = [os.path.join(REPO, "oracle", "_ref")]
 
 
 def ensure_pytensor() -> str:
@@ -24,8 +24,8 @@ def ensure_pytensor() -> str:
                 break
         else:
             raise ImportError(
-                "pytensor (the host framework) is not importable; run `bash oracle/build_ref.sh` to build "
-                "baseline/_ref from the reference checkout"
+                "pytensor (the host framework) is not importable; run `bash oracle/build_ref.sh <pytensor checkout>` "
+                "to build oracle/_ref"
             )
     # a writable compile dir for the host's C linker (used by the oracle; the CUDA backend does not need it)
     if "PYTENSOR_FLAGS" not in os.environ or "base_compiledir" not in os.environ.get("PYTENSOR_FLAGS", ""):

@@ -1,5 +1,6 @@
 """Build-time kernel cache warm-up: trace the BASELINE workloads in trace-only mode (runtime/lib.py TRACE_ONLY) so that
-every NVRTC kernel they launch is compiled for sm_100a into `pytensor_b200/_kcache/` on the CPU-only build box."""
+every NVRTC kernel they launch is compiled for sm_100a, without a GPU, into the cache `__graft_entry__.build()` points
+PTK_KCACHE at (`pytensor_b200/_kcache/`)."""
 
 from __future__ import annotations
 

@@ -2,22 +2,31 @@
 
 The reference compiles one C++ module per Apply node with g++ and caches it on disk keyed by op/type signature
 (pytensor/link/c/cmodule.py:612 ModuleCache, :1181-1260 module_from_key).  The B200 analogue: one sm_100a cubin per
-generated kernel source, cached in memory per process and on disk (in-tree `_kcache/`, so that cubins built by
-`__graft_entry__.build()` travel to the GPU box) keyed by the SHA-256 of (source, options).
+generated kernel source, cached in memory per process and on disk keyed by the SHA-256 of (source, options).  On disk,
+the cubins `__graft_entry__.build()` compiled into the package's `_kcache/` are read; kernels compiled at run time are
+written to a per-user directory under the system's temporary directory, so that running never writes into the source
+tree (which may be read-only).  `PTK_KCACHE` replaces both with one directory that is read and written (`build()` points
+it at `_kcache/`).
 """
 
 from __future__ import annotations
 
 import ctypes
+import functools
 import hashlib
 import os
+import stat
+import tempfile
 import threading
 
 from . import lib as _lib
 
-CACHE_DIR = os.environ.get(
-    "PTK_KCACHE", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "_kcache")
-)
+if "PTK_KCACHE" in os.environ:
+    CACHE_DIR = os.environ["PTK_KCACHE"]
+    READ_DIRS: tuple[str, ...] = (CACHE_DIR,)
+else:
+    CACHE_DIR = os.path.join(tempfile.gettempdir(), f"ptk_kcache_{os.getuid()}")
+    READ_DIRS = (os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "_kcache"), CACHE_DIR)
 
 _lock = threading.Lock()
 _cubins: dict[str, bytes] = {}
@@ -33,6 +42,21 @@ def _key(src: str, opts: tuple[str, ...]) -> str:
     return h.hexdigest()[:32]
 
 
+@functools.cache
+def _cache_dir_ok() -> bool:
+    """Whether CACHE_DIR may be read and written.  The default one sits in a directory where every user can create paths
+    and cache keys are predictable, so a cubin another user planted there would be loaded in place of ours: it is used
+    only as a real directory (not a link) that this user owns and that no one else can write to."""
+    if "PTK_KCACHE" in os.environ:
+        return True
+    try:
+        os.makedirs(CACHE_DIR, mode=0o700, exist_ok=True)
+        st = os.lstat(CACHE_DIR)
+    except OSError:
+        return False
+    return stat.S_ISDIR(st.st_mode) and st.st_uid == os.getuid() and not st.st_mode & 0o022
+
+
 def compile_cubin(src: str, opts: tuple[str, ...] = ()) -> tuple[str, bytes]:
     """Source -> (key, cubin bytes). Needs no GPU (NVRTC cross-compiles), so it also runs in the CPU-only build check."""
     key = _key(src, opts)
@@ -40,14 +64,16 @@ def compile_cubin(src: str, opts: tuple[str, ...] = ()) -> tuple[str, bytes]:
         if key in _cubins:
             stats["mem_hits"] += 1
             return key, _cubins[key]
+    for d in READ_DIRS:
+        cached = os.path.join(d, key + ".cubin")
+        if (d != CACHE_DIR or _cache_dir_ok()) and os.path.exists(cached):
+            with open(cached, "rb") as f:
+                data = f.read()
+            with _lock:
+                _cubins[key] = data
+                stats["disk_hits"] += 1
+            return key, data
     path = os.path.join(CACHE_DIR, key + ".cubin")
-    if os.path.exists(path):
-        with open(path, "rb") as f:
-            data = f.read()
-        with _lock:
-            _cubins[key] = data
-            stats["disk_hits"] += 1
-        return key, data
     L = _lib.load_library()
     cubin = ctypes.c_void_p()
     size = ctypes.c_size_t()
@@ -64,6 +90,8 @@ def compile_cubin(src: str, opts: tuple[str, ...] = ()) -> tuple[str, bytes]:
     data = ctypes.string_at(cubin.value, size.value)
     L.ptk_free(cubin)
     try:
+        if not _cache_dir_ok():
+            raise OSError(f"not a private directory: {CACHE_DIR}")
         os.makedirs(CACHE_DIR, exist_ok=True)
         tmp = path + f".tmp{os.getpid()}"
         with open(tmp, "wb") as f:

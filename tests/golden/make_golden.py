@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Generate tests/golden/<case>.npz: inputs + the outputs of the UNMODIFIED reference executing the graph through its C
-linker (mode="CVM").  Run in the build container (the reference lives in baseline/_ref there):
+linker (mode="CVM").  Run after `__graft_entry__.build()` (it builds the reference into oracle/_ref):
     python tests/golden/make_golden.py
 The fixtures pin (a) the CUDA backend on the GPU box without needing the reference there, and (b) oracle/numpy_port.py.
 """
